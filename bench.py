@@ -4,6 +4,8 @@ on the host CPU.
 
   python bench.py --gpus N --steps K --warmup W            our engine (libpn2_b200.so)
   python bench.py --impl reference --steps K --warmup W    reference path on the host cores
+  python bench.py ... --dump-outputs DIR                   also write what the last timed step computed
+                                                           to DIR/<name>.npy
 
 A "step" is one full training step of the reference's SSG network (model.py:22-161 +
 train.py:387-388): 4 SA + 4 FP layers + head, weighted CE loss, backward, Adam -- on a batch of
@@ -11,10 +13,11 @@ synthetic clouds with semantic.json's hyper-parameters (BASELINE.json configs[1]
 At N>1 every rank owns --batch clouds (weak scaling) and the step ends with ONE NCCL all-reduce
 over the flat gradient buffer.
 
-Timing: W warm-up steps, then K steps timed with CUDA events on the launching stream, an L2
-flush (256 MB write) between timed steps (outside the events), barrier + synchronize on both
-sides, MAX over ranks.  `value` has the inputs resident in HBM; `e2e` repeats the K steps
-through the same public API with pinned-host inputs copied in and the loss read back each step.
+Timing: W warm-up steps, then K steps timed with CUDA events on the launching stream, each from
+the freshly initialised model (restored, like the L2 flush (256 MB write) between timed steps,
+outside the events), barrier + synchronize on both sides, MAX over ranks.  `value` has the
+inputs resident in HBM; `e2e` repeats the K steps through the same public API with pinned-host
+inputs copied in and the loss read back each step.
 """
 import argparse
 import json
@@ -389,12 +392,31 @@ def fused_chain_bytes(b):
     return tot
 
 
+def step_state(trainer):
+    """The tensors a training step reads and updates besides its batch: weights, Adam moments, dropout counter,
+    BatchNorm moving statistics."""
+    return [trainer.flat, trainer.m, trainer.v, trainer._seed_dev] + trainer._moving()
+
+
+def dump_outputs(out_dir, trainer, loss):
+    """What the last timed step computed, as float32 .npy files: the loss it returned, the gradient it took, the
+    weights after its optimizer update and the BatchNorm moving statistics it updated.  Same arguments, same
+    seeded inputs, same starting state: two runs or two builds can be compared file by file."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.reshape(1), "grads": trainer.grads, "weights": trainer.flat,
+              "bn_moving_stats": torch.cat([t.reshape(-1) for t in trainer._moving()])}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
     import pn2_b200
     from pn2_b200 import _ffi
     from pn2_b200.train_step import Trainer
+    from pn2_b200.util import tf_util
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -425,7 +447,15 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    trainer.step(d_pc, d_lab, d_w)  # creates + flattens the variables
+    # Every timed step starts from the freshly initialised model: one pass that updates nothing creates the
+    # variables, and their state is put back before each timed step.  A step is deterministic up to the order
+    # of its fp32 atomics, but training on compounds that (Adam moves every weight whose gradient is near zero
+    # by a whole learning rate, whichever way the rounding tipped its sign), so a timed step that continued
+    # the warm-up's training would compute something different in every run.
+    with tf_util.frozen_moving_stats():
+        trainer.forward_backward(d_pc, d_lab, d_w)
+    start_count, start = trainer.step_count, [t.clone() for t in step_state(trainer)]
+    trainer.step(d_pc, d_lab, d_w)
     trainer.step(d_pc, d_lab, d_w)
     use_graph = (not args.no_graph) and trainer.capture(d_pc, d_lab, d_w)
     if not use_graph and not args.no_graph:
@@ -444,9 +474,11 @@ def run_ours(args):
     calls0 = _ffi.launches
     barrier()
     for i in range(args.steps):
+        trainer.step_count = start_count
+        torch._foreach_copy_(step_state(trainer), start)
         flush.zero_()
         ev[i][0].record()
-        step_fn(*dev_batches[i % NBATCH])
+        loss = step_fn(*dev_batches[i % NBATCH])
         ev[i][1].record()
     barrier()
     calls = _ffi.launches - calls0
@@ -454,6 +486,8 @@ def run_ours(args):
         calls = args.steps * (trainer.launches_per_replay + 1)
     ms = sum(a.elapsed_time(bb) for a, bb in ev)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, loss)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -629,6 +663,8 @@ def run_ours(args):
                        "wgrad_stream_sms": trainer.wgrad_sms,
                        "batches": "%d distinct synthetic batches rotated step by step (resident in HBM for value, "
                                   "pinned host memory for e2e)" % NBATCH,
+                       "start_state": "every step of value starts from the freshly initialised model "
+                                      "(restored outside the events)",
                        "geometry_ahead": ("every replay = dense stage of the current batch + sampling / neighbour "
                                           "search of the next batch on a second stream of the same graph; K steps "
                                           "run K of each") if (ahead and use_graph) else False,
@@ -655,7 +691,7 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=16, help="clouds per GPU")
@@ -667,7 +703,13 @@ def main():
                          "one batch ahead on a second stream")
     ap.add_argument("--no-extra", action="store_true",
                     help="skip the config-1 row and the 6-feature-channel line (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the engine's timed step computed: --impl ours only")
     if args.impl == "reference":
         run_reference(args)
     else:

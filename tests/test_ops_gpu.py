@@ -1,10 +1,12 @@
 """GPU parity: every tf_ops entry point, called through the Python op surface -> ctypes ->
 C ABI -> sm_100a kernels, against the CPU oracle (bit-exact for indices and copies, 1e-5 abs
-for interpolation) and against the reference's own CUDA kernels (oracle/_ref)."""
+for interpolation) and against what the reference's own CUDA kernels returned on the same inputs
+(tests/golden/reference_kernels.*, written by tests/golden/make_reference_golden.py from the
+functions named *_reference_inputs / *_REFERENCE_CASES below)."""
 import numpy as np
 import pytest
 
-from _util import RefKernels, golden, golden_inputs, rng_cloud, to_cuda
+from _util import assert_reference, assert_reference_close, golden, golden_inputs, rng_cloud, to_cuda
 
 pytestmark = pytest.mark.gpu
 
@@ -61,16 +63,17 @@ def test_fps_properties_full_size(ops):
     assert all(sel[i] >= sel[i + 1] - 1e-9 for i in range(len(sel) - 1))
 
 
+def fps_reference_inputs():
+    """(key, cloud, npoint) of the FPS comparisons with the reference's kernel."""
+    for b, n, m in [(2, 1024, 256), (16, 8192, 1024), (3, 5000, 333)]:
+        yield "fps_%d_%d_%d" % (b, n, m), rng_cloud(5 + n, b, n), m
+    yield "fps_lattice_2_3000_400", np.random.RandomState(3).randint(0, 5, (2, 3000, 3)).astype(np.float32), 400
+
+
 def test_fps_matches_reference_kernel(ops):
     ts, _, _, _ = ops
-    ref = RefKernels()
-    for b, n, m in [(2, 1024, 256), (16, 8192, 1024), (3, 5000, 333)]:
-        x = to_cuda(rng_cloud(5 + n, b, n))
-        np.testing.assert_array_equal(ts.farthest_point_sample(m, x).cpu().numpy(),
-                                      ref.fps(x, m).cpu().numpy())
-    g = to_cuda(np.random.RandomState(3).randint(0, 5, (2, 3000, 3)).astype(np.float32))
-    np.testing.assert_array_equal(ts.farthest_point_sample(400, g).cpu().numpy(),
-                                  ref.fps(g, 400).cpu().numpy())
+    for key, x, m in fps_reference_inputs():
+        assert_reference(key, ts.farthest_point_sample(m, to_cuda(x)))
 
 
 def test_gather_point_and_grad(ops):
@@ -142,17 +145,20 @@ def test_query_ball_boundary_radius(ops):
         np.testing.assert_array_equal(idx.cpu().numpy(), eidx)
 
 
-def test_query_ball_matches_reference_kernel(ops):
-    _, tg, _, _ = ops
-    ref = RefKernels()
+def ball_reference_inputs():
+    """(key, radius, nsample, cloud, queries) of the ball-query comparisons with the reference's kernel."""
     for b, n, m, radius, ns in [(2, 1024, 256, 0.2, 32), (16, 8192, 1024, 0.1, 32),
                                 (4, 2048, 512, 0.25, 64)]:
-        x1 = to_cuda(rng_cloud(21 + n, b, n))
-        x2 = x1[:, :m].contiguous()
-        idx, cnt = tg.query_ball_point(radius, ns, x1, x2)
-        ridx, rcnt = ref.query_ball_point(radius, ns, x1, x2)
-        np.testing.assert_array_equal(cnt.cpu().numpy(), rcnt.cpu().numpy())
-        np.testing.assert_array_equal(idx.cpu().numpy(), ridx.cpu().numpy())
+        x1 = rng_cloud(21 + n, b, n)
+        yield "ball_%d_%d_%d_%g_%d" % (b, n, m, radius, ns), radius, ns, x1, np.ascontiguousarray(x1[:, :m])
+
+
+def test_query_ball_matches_reference_kernel(ops):
+    _, tg, _, _ = ops
+    for key, radius, ns, x1, x2 in ball_reference_inputs():
+        idx, cnt = tg.query_ball_point(radius, ns, to_cuda(x1), to_cuda(x2))
+        assert_reference(key + "_cnt", cnt)
+        assert_reference(key + "_idx", idx)
 
 
 def test_query_ball_validation(ops):
@@ -287,14 +293,6 @@ def test_three_interpolate_grad_check_like_reference(ops):
         assert abs(fd - an) / max(1.0, abs(an)) < 1e-4
 
 
-def _ref_kernels():
-    from _util import RefKernels
-    try:
-        return RefKernels()
-    except FileNotFoundError:
-        pytest.skip("oracle/_ref not built")
-
-
 def _selection_cases():
     rs = np.random.RandomState(9)
     nan = rs.randint(0, 4, (1, 12, 150)).astype(np.float32)
@@ -311,7 +309,7 @@ def _selection_cases():
 @pytest.mark.parametrize("k", [1, 16, 128])
 def test_select_top_k_matches_oracle_and_reference_kernel(ops, name, k):
     """The WHOLE output rows (first k and the permuted tail) against the C oracle and against the
-    reference's own selection_sort_gpu running on the same GPU -- ties, NaN and inf included."""
+    reference's own selection_sort_gpu -- ties, NaN and inf included."""
     _, tg, _, orc = ops
     d = np.ascontiguousarray(_selection_cases()[name], np.float32)
     if k > d.shape[2] and d.shape[2] > 128:
@@ -321,13 +319,8 @@ def test_select_top_k_matches_oracle_and_reference_kernel(ops, name, k):
     ei, eo = orc.select_top_k(k, d)
     np.testing.assert_array_equal(outi.cpu().numpy(), ei)
     np.testing.assert_array_equal(out.cpu().numpy().view(np.uint32), eo.view(np.uint32))
-    ri, ro = _ref_kernels().selection_sort(k, dd)
-    assert bool((ri == outi).all()) and bool((ro.view(torch_i32()) == out.view(torch_i32())).all())
-
-
-def torch_i32():
-    import torch
-    return torch.int32
+    assert_reference("select_%s_k%d_idx" % (name, k), outi)
+    assert_reference("select_%s_k%d_val" % (name, k), out)
 
 
 def _sqdist_matrix(x1, x2):
@@ -340,15 +333,14 @@ def _sqdist_matrix(x1, x2):
     return acc
 
 
-@pytest.mark.parametrize("b,n,m,k,c,kind", [(2, 1024, 256, 32, 3, "uniform"), (32, 512, 128, 32, 3, "uniform"),
-                                           (1, 8192, 100, 64, 3, "uniform"), (2, 300, 50, 16, 3, "lattice"),
-                                           (1, 200, 30, 128, 3, "duplicates"), (2, 400, 60, 8, 5, "uniform"),
-                                           (1, 64, 10, 64, 2, "lattice")])
-def test_knn_point_fused_matches_oracle_and_reference_selection(ops, b, n, m, k, c, kind):
-    """knn_point (one fused kernel, no (b,m,n) tensor) == the oracle restatement of tf_grouping.py:64-89 ==
-    the reference's own selection kernel applied to the fp32 distance matrix; (32,512)/(32,128), k=32 is the
-    reference's smoke-test shape (test_tf_ops.py:9-24)."""
-    _, tg, _, orc = ops
+KNN_REFERENCE_CASES = [(2, 1024, 256, 32, 3, "uniform"), (32, 512, 128, 32, 3, "uniform"),
+                       (1, 8192, 100, 64, 3, "uniform"), (2, 300, 50, 16, 3, "lattice"),
+                       (1, 200, 30, 128, 3, "duplicates"), (2, 400, 60, 8, 5, "uniform"),
+                       (1, 64, 10, 64, 2, "lattice")]
+
+
+def knn_reference_inputs(b, n, m, k, c, kind):
+    """(key, x1, x2) of a knn_point case; the reference's selection kernel ran on _sqdist_matrix(x1, x2)."""
     rs = np.random.RandomState(n + k)
     if kind == "uniform":
         x1, x2 = rs.random_sample((b, n, c)), rs.random_sample((b, m, c))
@@ -357,13 +349,23 @@ def test_knn_point_fused_matches_oracle_and_reference_selection(ops, b, n, m, k,
     else:
         x1 = np.repeat(rs.random_sample((b, n // 4, c)), 4, 1)
         x2 = x1[:, :m] + 0.0
-    x1, x2 = np.ascontiguousarray(x1, np.float32), np.ascontiguousarray(x2, np.float32)
+    key = "knn_%d_%d_%d_%d_%d_%s" % (b, n, m, k, c, kind)
+    return key, np.ascontiguousarray(x1, np.float32), np.ascontiguousarray(x2, np.float32)
+
+
+@pytest.mark.parametrize("b,n,m,k,c,kind", KNN_REFERENCE_CASES)
+def test_knn_point_fused_matches_oracle_and_reference_selection(ops, b, n, m, k, c, kind):
+    """knn_point (one fused kernel, no (b,m,n) tensor) == the oracle restatement of tf_grouping.py:64-89 ==
+    the reference's own selection kernel applied to the fp32 distance matrix; (32,512)/(32,128), k=32 is the
+    reference's smoke-test shape (test_tf_ops.py:9-24)."""
+    _, tg, _, orc = ops
+    key, x1, x2 = knn_reference_inputs(b, n, m, k, c, kind)
     val, idx = tg.knn_point(k, to_cuda(x1), to_cuda(x2))
     ev, ei = orc.knn_point(k, x1, x2)
     np.testing.assert_array_equal(idx.cpu().numpy(), ei)
     np.testing.assert_array_equal(val.cpu().numpy().view(np.uint32), ev.view(np.uint32))
-    ri, ro = _ref_kernels().selection_sort(k, to_cuda(_sqdist_matrix(x1, x2)))
-    assert bool((ri[:, :, :k] == idx).all()) and bool((ro[:, :, :k] == val).all())
+    assert_reference(key + "_idx", idx)  # the first k columns of the reference's selection
+    assert_reference(key + "_val", val)
 
 
 def test_knn_point_validation(ops):
@@ -375,27 +377,34 @@ def test_knn_point_validation(ops):
         tg.knn_point(51, x, x)
 
 
-def test_gather_and_group_match_reference_kernels(ops):
-    """gather_point / group_point and their gradients against the reference's own kernels on the same GPU
-    (exact for the gathers; the scatter-adds use fp32 atomics on both sides: 1e-5)."""
-    import torch
-    ts, tg, _, _ = ops
-    ref = _ref_kernels()
+def gather_group_reference_inputs():
+    """(cloud, gradient of the 256 gathered points, [(c, points, gradient of the grouped points)]); the gathers
+    take FPS(256) of the cloud, the groups the ball query (0.2, 32) around those points."""
     rs = np.random.RandomState(4)
-    x = to_cuda(rs.random_sample((16, 8192, 3)).astype(np.float32))
+    x = rs.random_sample((16, 8192, 3)).astype(np.float32)
+    g = rs.normal(size=(16, 256, 3)).astype(np.float32)
+    groups = [(c, rs.random_sample((16, 8192, c)).astype(np.float32),
+               rs.normal(size=(16, 256, 32, c)).astype(np.float32)) for c in (3, 16, 67)]
+    return x, g, groups
+
+
+def test_gather_and_group_match_reference_kernels(ops):
+    """gather_point / group_point and their gradients against the reference's own kernels: exact for the
+    gathers and for gather_point's gradient (FPS indices are distinct: one addition per element); group_point's
+    gradient adds up to 32 contributions per element with fp32 atomics on both sides: 2e-5."""
+    ts, tg, _, _ = ops
+    x, g, groups = gather_group_reference_inputs()
+    x = to_cuda(x)
     fps = ts.farthest_point_sample(256, x)
-    assert bool((ts.gather_point(x, fps) == ref.gather_point(x, fps)).all())
-    g = to_cuda(rs.normal(size=(16, 256, 3)).astype(np.float32))
-    np.testing.assert_allclose(ts.gather_point_grad(x, fps, g).cpu().numpy(),
-                               ref.gather_point_grad(x, fps, g).cpu().numpy(), atol=1e-5)
+    assert_reference("gather_point", ts.gather_point(x, fps))
+    assert_reference("gather_point_grad", ts.gather_point_grad(x, fps, to_cuda(g)))
     new = ts.gather_point(x, fps)
     idx, _ = tg.query_ball_point(0.2, 32, x, new)
-    for c in (3, 16, 67):
-        pts = to_cuda(rs.random_sample((16, 8192, c)).astype(np.float32))
-        assert bool((tg.group_point(pts, idx) == ref.group_point(pts, idx)).all())
-        go = to_cuda(rs.normal(size=(16, 256, 32, c)).astype(np.float32))
-        np.testing.assert_allclose(tg.group_point_grad(pts, idx, go).cpu().numpy(),
-                                   ref.group_point_grad(pts, idx, go).cpu().numpy(), atol=2e-5, rtol=1e-5)
+    for c, pts, go in groups:
+        pts = to_cuda(pts)
+        assert_reference("group_point_c%d" % c, tg.group_point(pts, idx))
+        assert_reference_close("group_point_grad_c%d" % c, tg.group_point_grad(pts, idx, to_cuda(go)),
+                               atol=2e-5, rtol=1e-5)
 
 
 # ---------------------------------------------------------------- prob_sample (SURVEY 8f-1)
@@ -431,22 +440,22 @@ def test_prob_sample_matches_oracle(ops, b, n, m):
     np.testing.assert_array_equal(cdf.cpu().numpy().view(np.uint32), orc.cumsum(p).view(np.uint32))
 
 
+PROB_REFERENCE_CASES = [(1, 5, 8192), (2, 8193, 500), (3, 20000, 2000), (32, 1000, 100)]
+
+
 def test_prob_sample_matches_reference_kernel(ops):
-    """Against the reference's own cumsumKernel + binarysearchKernel running on this GPU."""
+    """Against the reference's own cumsumKernel + binarysearchKernel: indices and CDF."""
     import torch
     from pn2_b200._ffi import F32, call, ptr
     ts, _, _, _ = ops
-    ref = RefKernels()
-    for b, n, m in [(1, 5, 8192), (2, 8193, 500), (3, 20000, 2000), (32, 1000, 100)]:
+    for b, n, m in PROB_REFERENCE_CASES:
         p, r = _prob_inputs(b, n, m)
         pc, rc = to_cuda(p), to_cuda(r)
-        exp_idx, exp_cdf = ref.prob_sample(pc, rc)
         got = ts.prob_sample(pc, rc)
-        np.testing.assert_array_equal(got.cpu().numpy(), exp_idx.cpu().numpy())
+        assert_reference("prob_%d_%d_%d_idx" % (b, n, m), got)
         cdf = torch.empty_like(pc)
         call("pn2_cumsum", b, n, ptr(pc, F32), ptr(cdf, F32))
-        np.testing.assert_array_equal(cdf.cpu().numpy().view(np.uint32),
-                                      exp_cdf.cpu().numpy().view(np.uint32))
+        assert_reference("prob_%d_%d_%d_cdf" % (b, n, m), cdf)
 
 
 def test_prob_sample_like_reference_test(ops):
@@ -593,9 +602,7 @@ def test_fps_cluster_tie_order(ops):
 
 
 def test_fps_cluster_matches_reference_kernel(ops):
-    ref = RefKernels()
-    x = to_cuda(rng_cloud(77, 2, 30000))
-    np.testing.assert_array_equal(_fps_cluster(x, 256).cpu().numpy(), ref.fps(x, 256).cpu().numpy())
+    assert_reference("fps_cluster_2_30000_256", _fps_cluster(to_cuda(rng_cloud(77, 2, 30000)), 256))
 
 
 # ------------------------------------------------------------- committed golden fixtures
