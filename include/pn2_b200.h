@@ -411,6 +411,22 @@ int pn2_box_sample(int B, long P, int num_point, int feat, const double *points,
                    float *out_weights, int *out_index, int *out_count, pn2_stream_t s);
 unsigned pn2_box_sample_key(unsigned long long seed, int sample, long i);
 
+/* ---- group 4: evaluation --------------------------------------------------------------------------------
+ * replaces ConfusionMatrix.increment / increment_from_list   util/metric.py:7-83
+ *          fed by np.argmax over the host copy of pred        train.py:246-251 (and :307-312, predict.py:90)
+ * The logits never leave the device and nothing synchronises the host, so both calls can be captured in a CUDA
+ * graph.  cm (C*C, row = ground truth, column = prediction) and skipped are uint64 accumulators the caller
+ * zeroes; calls accumulate.  1 <= C <= 128 (PN2_EUNSUPPORTED above). */
+/* per row r < rows: pd = arg-max of logits[r, 0:C] with numpy's rule (first maximum; the first NaN wins);
+ * if 0 <= labels[r] < C: cm[labels[r]*C + pd] += 1, else *skipped += 1.  pred_out (rows) int32 or NULL. */
+int pn2_confusion_from_logits(long rows, int C, const float *logits, const int *labels,
+                              unsigned long long *cm, unsigned long long *skipped, int *pred_out,
+                              pn2_stream_t s);
+/* the same for label pairs; a pair with gt or pd outside [0,C) is skipped (sklearn's
+ * confusion_matrix(labels=range(C)), which metric.py:25-30 calls) */
+int pn2_confusion_from_labels(long n, int C, const int *gt, const int *pd,
+                              unsigned long long *cm, unsigned long long *skipped, pn2_stream_t s);
+
 #ifdef __cplusplus
 }
 #endif

@@ -23,7 +23,7 @@ def install_reference_aliases(include_model=True):
     model.py (see compat/tensorflow.py)."""
     from . import tf_ops, util, model, predict
     from .tf_ops import tf_grouping, tf_interpolate, tf_sampling
-    from .util import pointnet_util, tf_util
+    from .util import metric, pointnet_util, tf_util
     sys.modules.setdefault("tf_ops", tf_ops)
     sys.modules.setdefault("tf_ops.tf_sampling", tf_sampling)
     sys.modules.setdefault("tf_ops.tf_grouping", tf_grouping)
@@ -31,6 +31,7 @@ def install_reference_aliases(include_model=True):
     sys.modules.setdefault("util", util)
     sys.modules.setdefault("util.tf_util", tf_util)
     sys.modules.setdefault("util.pointnet_util", pointnet_util)
+    sys.modules.setdefault("util.metric", metric)
     if include_model:
         sys.modules.setdefault("model", model)      # the reference's top-level `import model`
         sys.modules.setdefault("predict", predict)  # `from predict import Predictor`

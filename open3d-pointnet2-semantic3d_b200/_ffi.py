@@ -89,6 +89,8 @@ SIGNATURES = {
                        ctypes.c_double, _ull, _vp, _vp, _vp, _vp, _vp, _vp],
     "pn2_box_sample_key": [_ull, _i, _l],
     "pn2_adam_step": [_l, _vp, _vp, _vp, _vp, _f, _f, _f, _f, _i, _f, _vp],
+    "pn2_confusion_from_logits": [_l, _i, _vp, _vp, _vp, _vp, _vp, _vp],
+    "pn2_confusion_from_labels": [_l, _i, _vp, _vp, _vp, _vp, _vp],
 }
 _RESTYPE = {"pn2_strerror": ctypes.c_char_p, "pn2_last_cuda_error": ctypes.c_char_p,
             "pn2_ball_threshold": ctypes.c_float, "pn2_linear_workspace_bytes": ctypes.c_long,

@@ -4,6 +4,8 @@
   Trainer.step: forward, loss, backward, Adam            train.py:387-388, 225-244
   data parallelism: batch sharded across ranks, ONE NCCL all-reduce over the flat gradient
   buffer per step (SURVEY.md section 8e); BatchNorm statistics stay per replica.
+  Trainer.evaluate: eval-mode forward + loss + confusion      train.py:263-330 (sess.run([loss, pred]), :296-312)
+  Trainer.train_confusion: confusion of every training pass  train.py:234-251
 
 Stream discipline: a Trainer owns ONE CUDA stream and issues every launch of its replica on it --
 the eager passes, the CUDA-graph capture and the replays alike.  The autograd engine ties each
@@ -37,6 +39,7 @@ import torch.distributed as dist
 from . import _ffi, model
 from ._ffi import F32, call, ptr
 from .util import pointnet_util, tf_util
+from .util.metric import ConfusionMatrix
 
 
 def get_learning_rate(step, params):
@@ -112,6 +115,16 @@ class Trainer:
         self.wgrad_sms = int(os.environ.get("PN2_WGRAD_SMS", "64")) if wgrad_sms is None else int(wgrad_sms)
         self._wstream = torch.cuda.Stream(device=self.device) if self.wgrad_sms > 0 else None
         self._side = torch.cuda.Stream(device=self.device) if self.geometry_ahead else None
+        # a util.metric.ConfusionMatrix: every training pass adds the confusion of its training-mode logits
+        # (dropout applied, the train op's `pred` of train.py:234-251); part of the captured step graph, so setting
+        # or clearing it re-captures on the next step_graph
+        self.train_confusion = None
+        self._graph_train_confusion = None
+        # evaluate(): one graph per batch shape (None = eager, the reason in _eval_capture_error); the pass counts
+        # into a trainer-owned matrix that the graph zeroes, so the caller's matrix is not baked into the graph
+        self._eval_graphs = {}
+        self._eval_cm = None
+        self._eval_capture_error = None
 
     # ---- variables ----------------------------------------------------------------------------
     def _ensure_flat(self):
@@ -161,6 +174,8 @@ class Trainer:
                 finally:
                     if os.environ.get("PN2_AHEAD_SCOPE", "fwd") != "step":
                         self._sm_budget(0)
+                if self.train_confusion is not None:
+                    self.train_confusion.increment_from_logits(pred.detach(), labels.to(torch.int32).contiguous())
                 self.store.zero_grad()
                 loss = model.get_loss(pred, labels, smpw)
                 if self.wgrad_sms > 0:  # weight gradients next to the rest of the backward pass (util/tf_util.py)
@@ -291,6 +306,9 @@ class Trainer:
                         if d.data_ptr() != s.data_ptr():
                             d.copy_(s)
                 static = self._static
+                # the warm-up passes and the validation replay count too: their counts are undone below
+                cm = self.train_confusion
+                keep_cm = None if cm is None else cm._counts.clone()
                 with tf_util.frozen_moving_stats():
                     for _ in range(2):  # every kernel / workspace / gradient buffer exists
                         self._fb(*static, ahead=ahead)
@@ -310,9 +328,12 @@ class Trainer:
                 self.stream.synchronize()
                 for t, k in zip(self._moving(), keep):
                     t.copy_(k)
+                if cm is not None:
+                    cm._counts.copy_(keep_cm)
                 self._static_loss = loss
                 self._graph = g
                 self._graph_bn_decay = get_bn_decay(self.step_count, self.params)
+                self._graph_train_confusion = cm
         except Exception as e:  # noqa: BLE001 - any capture failure means eager mode
             import traceback
             self._graph = None
@@ -385,7 +406,8 @@ class Trainer:
                 raise ValueError("geometry_ahead: call prime(first_batch) before the first step_graph(next_batch)")
             if any(a.shape != b.shape for a, b in zip(self._static, src)):
                 raise ValueError("geometry_ahead needs a fixed batch shape")
-            if self._graph is None or get_bn_decay(self.step_count, self.params) != self._graph_bn_decay:
+            if self._graph is None or get_bn_decay(self.step_count, self.params) != self._graph_bn_decay or \
+                    self.train_confusion is not self._graph_train_confusion:
                 if not self.capture(*self._static):
                     raise _ffi.Pn2Error("geometry_ahead needs graph mode; capture failed: %s" % self._capture_error)
             inputs = self._next
@@ -395,6 +417,7 @@ class Trainer:
                     torch.cuda.current_stream(self.device).wait_event(self._staged_event)
                 return self.step(*src)
             if get_bn_decay(self.step_count, self.params) != self._graph_bn_decay or \
+                    self.train_confusion is not self._graph_train_confusion or \
                     any(a.shape != b.shape for a, b in zip(self._static, src)):
                 if staged:
                     torch.cuda.current_stream(self.device).wait_event(self._staged_event)
@@ -418,3 +441,81 @@ class Trainer:
             self._apply_gradients()
         caller.wait_stream(self.stream)
         return self._static_loss
+
+    # ---- evaluation: eval_one_epoch's sess.run([loss, pred]) (train.py:296-312) -------------------------
+    def _eval_pass(self, point_cloud, labels, smpw):
+        """Eval-mode forward (moving-average BatchNorm, no dropout) + loss, no backward; the confusion of the
+        logits goes to self._eval_cm, which the pass zeroes first.  Geometry is computed inline: a geometry-ahead
+        tape is neither read nor advanced.  Weights, moving statistics and the dropout counter are only read."""
+        tf_util.set_default_store(self.store)
+        tf_util.zero_arena.reset(self.device)
+        fresh = self.store.images_fresh
+        try:
+            self.store.prepare_images()  # the weights change between calls: part of the pass (and of its graph)
+            with torch.no_grad(), pointnet_util.replay_geometry(None):
+                pred, _ = model.get_model(point_cloud, False, self.num_class, self.params)
+                loss = model.get_loss(pred, labels, smpw)
+                self._eval_cm.reset()
+                self._eval_cm.increment_from_logits(pred.contiguous(), labels.to(torch.int32).contiguous())
+        finally:
+            tf_util.zero_arena.disarm()
+            self.store.images_fresh = fresh
+        return loss
+
+    def _capture_eval(self, src):
+        """-> (graph, static inputs, static loss) of the eval pass for this batch shape, or None (eager mode;
+        the reason is kept in self._eval_capture_error)."""
+        static = [t.clone() for t in src]
+        try:
+            self._eval_pass(*static)  # every kernel attribute / buffer exists before the capture
+            self.stream.synchronize()
+            gc.collect()
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, stream=self.stream, capture_error_mode="thread_local"):
+                loss = self._eval_pass(*static)
+            g.replay()  # validation replay (raises on a broken graph); the pass has no side effect to undo
+            self.stream.synchronize()
+            return g, static, loss
+        except Exception as e:  # noqa: BLE001 - any capture failure means eager mode
+            import traceback
+            self._eval_capture_error = repr(e) + " | " + traceback.format_exc()
+            try:
+                torch.cuda.synchronize()
+            except Exception:  # noqa: BLE001
+                pass
+            return None
+
+    def evaluate(self, point_cloud, labels, smpw, confusion=None, graph=True):
+        """Eval-mode loss of one batch (0-dim CUDA tensor, this call's own); with ``confusion`` (a
+        util.metric.ConfusionMatrix) the confusion of the eval logits is added to it.  Runs on the replica's
+        stream, by replay of a graph captured once per batch shape (``graph=False``: eager launches).  Leaves
+        every piece of training state as it was: weights, Adam moments, moving statistics, step and dropout
+        counters, the training graph and the geometry-ahead pipeline."""
+        if confusion is not None and confusion.num_classes != self.num_class:
+            raise ValueError("confusion has %d classes, the model %d" % (confusion.num_classes, self.num_class))
+        caller = torch.cuda.current_stream(self.device)
+        self.stream.wait_stream(caller)
+        with torch.cuda.stream(self.stream):
+            src = self._to_device(point_cloud, labels, smpw)
+            self._create_variables(src[0])
+            if self._eval_cm is None:
+                self._eval_cm = ConfusionMatrix(self.num_class, device=self.device)
+            entry = None
+            if graph:
+                key = tuple((tuple(t.shape), t.dtype) for t in src)
+                if key not in self._eval_graphs:
+                    self._eval_graphs[key] = self._capture_eval(src)
+                entry = self._eval_graphs[key]
+            if entry is not None:
+                g, static, static_loss = entry
+                for d, s in zip(static, src):
+                    d.copy_(s, non_blocking=True)
+                g.replay()
+                loss = static_loss.clone()  # the next replay overwrites static_loss
+            else:
+                loss = self._eval_pass(*src)
+            if confusion is not None:
+                confusion._counts.add_(self._eval_cm._counts)
+        loss.record_stream(caller)
+        caller.wait_stream(self.stream)
+        return loss
